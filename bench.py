@@ -461,6 +461,25 @@ def run_reference_fit(args, wl):
     return {"value": 1.0 / est, "unit": "iters/sec", "cores": threads, "kind": "reference", "sample": sample}
 
 
+DUMP_SCORE_ROWS = 1 << 20      # 8 MB of float64 scores (+ their row ids) whatever the workload's row count
+
+
+def dump_outputs(out_dir, tree, scores):
+    """What B200Booster.update() hands back in the last timed step (the tree: every split field, the leaf arrays) and the
+    training scores it leaves, as float64 .npy files.  Scores of more than DUMP_SCORE_ROWS rows are sampled at row ids
+    fixed by a seed, so that runs with the same arguments write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {f"tree_split_{k}": tree.splits[k] for k in tree.splits.dtype.names}
+    out.update(tree_leaf_value=tree.leaf_value, tree_leaf_weight=tree.leaf_weight, tree_leaf_count=tree.leaf_count,
+               tree_leaf_depth=tree.leaf_depth, tree_num_leaves=np.array([tree.num_leaves]))
+    rows = np.arange(len(scores))
+    if len(scores) > DUMP_SCORE_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(len(scores), DUMP_SCORE_ROWS, replace=False))
+    out.update(score_rows=rows, scores=scores[rows])
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -475,7 +494,14 @@ def main():
                     help="NOT the headline: train with use_quantized_grad=true, num_grad_quant_bins=Q (both arms)")
     ap.add_argument("--no-replicate", action="store_true",
                     help="N>1: keep one copy of the partition columns across the box (the split's owner pushes go-left bits)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the tree of the last timed step and the training scores (a fixed "
+                         "sample of rows) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of this repo's arm (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     rank, world, local = dist_env()
     wl = dict(WORKLOADS[args.workload])
@@ -609,6 +635,8 @@ def main():
         ms_total = L.timer_stop()
         barrier()
         wall = time.time() - t0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, t, B.scores())
     ms_total = max_over_ranks(ms_total)
     launches = L.kernel_launches - l0
     ms_per_step = ms_total / args.steps

@@ -70,39 +70,42 @@ def test_c2_full_split_sequence_matches_oracle(built_lib, const_hess):
     assert total >= 62
 
 
-def test_c2_first_tree_matches_the_compiled_reference(built_lib):
-    """The same C2 matrix through the UNMODIFIED reference library (oracle/_ref, LGBM_BoosterUpdateOneIterCustom with the
-    same gradients, serial col-wise deterministic CPU learner) and through the CUDA path: same split features, same
-    real-valued thresholds (bin upper bounds), same child counts, for every split of the first tree."""
-    import lightgbm_b200 as lgb
-    from oracle import refapi
-    if not refapi.available():
-        pytest.skip("oracle/_ref not built")
+def c2_reference_inputs():
+    """C2 bins, labels, first-iteration gradients, and the reference Dataset / Booster parameters of
+    test_c2_first_tree_matches_the_compiled_reference."""
     rows, cols, leaves = 1_000_000, 256, 63
     bins, y = _workload(rows, cols, 42)
     dsp = dict(max_bin=255, min_data_in_bin=1, enable_bundle="false", feature_pre_filter="false", verbosity=-1,
                num_threads=min(32, os.cpu_count() or 8))
-    ds = refapi.RefDatasetStreamed(lambda lo, hi: bins[lo:hi].astype(np.float32), rows, cols, y, dsp, block_rows=262144)
-    bst = refapi.RefBooster(ds, dict(dsp, objective="custom", num_leaves=leaves, min_data_in_leaf=20, learning_rate=1.0,
-                                     device_type="cpu", force_col_wise="true", deterministic="true"))
+    bp = dict(dsp, objective="custom", num_leaves=leaves, min_data_in_leaf=20, learning_rate=1.0, device_type="cpu",
+              force_col_wise="true", deterministic="true")
     g = (float(np.mean(y, dtype=np.float64)) - y).astype(np.float32)
     h = np.ones(rows, np.float32)
-    bst.update_custom(g, h)
-    ref = bst.trees()[0]
-    bst.free(); ds.free()
+    return bins, y, g, h, dsp, bp
+
+
+def test_c2_first_tree_matches_the_compiled_reference(built_lib):
+    """The same C2 matrix through the UNMODIFIED reference library (oracle/_ref, LGBM_BoosterUpdateOneIterCustom with the
+    same gradients, serial col-wise deterministic CPU learner; its tree is recorded in tests/golden/reference/c2_first_tree.npz)
+    and through the CUDA path: same split features, same real-valued thresholds (bin upper bounds), same child counts, for
+    every split of the first tree."""
+    import lightgbm_b200 as lgb
+    bins, y, g, h, _, bp = c2_reference_inputs()
+    leaves = bp["num_leaves"]
+    ref = np.load(os.path.join(ROOT, "tests", "golden", "reference", "c2_first_tree.npz"))
 
     L = lgb.B200TreeLearner(lgb.Config(num_leaves=leaves, min_data_in_leaf=20))
     L.init(lgb.Layout.identity(bins), is_constant_hessian=True)
     t = L.train(g, h)
-    assert t.num_leaves == ref.num_leaves == leaves
-    np.testing.assert_array_equal(t.splits["leaf"], ref.split_leaf())
-    np.testing.assert_array_equal(t.splits["feature"], ref.split_feature)
+    assert t.num_leaves == int(ref["num_leaves"]) == leaves
+    np.testing.assert_array_equal(t.splits["leaf"], ref["split_leaf"])
+    np.testing.assert_array_equal(t.splits["feature"], ref["split_feature"])
     # identity bins: value v has bin v, bin upper bound = v + 0.5 (bin.cpp: midpoints of consecutive distinct values)
-    np.testing.assert_allclose(ref.threshold, t.splits["threshold"] + 0.5, atol=1e-6)
-    np.testing.assert_array_equal(t.splits["left_count"] + t.splits["right_count"], ref.internal_count)
-    np.testing.assert_array_equal(t.leaf_count, ref.leaf_count)
-    np.testing.assert_allclose(t.splits["gain"], ref.split_gain, rtol=2e-5)     # the model text stores float32 gains
-    np.testing.assert_allclose(t.leaf_value, ref.leaf_value, rtol=1e-6, atol=1e-9)
+    np.testing.assert_allclose(ref["threshold"], t.splits["threshold"] + 0.5, atol=1e-6)
+    np.testing.assert_array_equal(t.splits["left_count"] + t.splits["right_count"], ref["internal_count"])
+    np.testing.assert_array_equal(t.leaf_count, ref["leaf_count"])
+    np.testing.assert_allclose(t.splits["gain"], ref["split_gain"], rtol=2e-5)     # the model text stores float32 gains
+    np.testing.assert_allclose(t.leaf_value, ref["leaf_value"], rtol=1e-6, atol=1e-9)
 
 
 def test_c3_shaped_2m_x_1024_matches_oracle(built_lib):
